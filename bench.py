@@ -2,6 +2,7 @@
 """bench.py — tokens/s of the llama2.zig decode hot path on B200, with its HBM roofline.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload ...]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -52,6 +53,7 @@ WORKLOADS = {
 }
 SYNTH_SEED = {"stories15M": 15, "stories110M": 110, "llama2-7B": 7}
 L2_FLUSH_BYTES = 256 << 20   # > 126 MB L2
+KV_SAMPLE = 1 << 20          # floats kept per cache by --dump-outputs
 SYNTH_DESC = "synthetic (counter-based N(0,s) weights, same generator on GPU and CPU; teacher-forced tokens)"
 
 
@@ -221,6 +223,35 @@ def run_reference_arm(args, rank, world):
 # ----------------------------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------------------------
+def step_outputs(t, positions, tokens, with_logits):
+    """What the last timed step computed, as its caller would read it back: the logits of its last
+    position (classifier output; single-GPU contexts only, a sharded context keeps them in per-rank
+    slices), the final hidden state x (before the final rmsnorm), and the key / value cache rows of
+    the positions it ran (float32), plus the token ids it returned (float64, exact).  Under teacher
+    forcing those ids are the forced input, not a result.  A cache larger than KV_SAMPLE floats is
+    reduced to a fixed, seeded sample so that a dump stays far below 64 MB."""
+    out = {"tokens": np.asarray(tokens, dtype=np.float64), "x": t.state("x")}
+    if with_logits:
+        out["logits"] = t.state("logits")
+    for name in ("key_cache", "value_cache"):
+        cache = t.state(name)                                  # [n_layers][seq_len][kv width]
+        per_layer = cache.size // t.ck.n_layers
+        filled = per_layer // t.ck.seq_len * positions
+        n = t.ck.n_layers * filled
+        idx = np.arange(n) if n <= KV_SAMPLE else np.sort(np.random.default_rng(0).integers(0, n, KV_SAMPLE))
+        out[name] = cache[idx // filled * per_layer + idx % filled]
+    return out
+
+
+def dump_outputs(dirname, outputs):
+    """DIR/<workload>_<name>.npy for every array of step_outputs.  Inputs are seeded, so two builds
+    run with the same arguments can be compared file for file."""
+    os.makedirs(dirname, exist_ok=True)
+    for workload, arrays in outputs.items():
+        for name, a in arrays.items():
+            np.save(os.path.join(dirname, f"{workload}_{name}.npy"), a)
+
+
 def kernel_source_sha():
     import hashlib
     h = hashlib.sha256()
@@ -322,11 +353,22 @@ def run_workload(workload, args, rank, world, dist, sync, flush, clock_index):
         data_desc = SYNTH_DESC
         forced = teacher_tokens(positions + 1, ck.vocab_size)[1:]
 
+    last = {}
+
     def device_run():
         t.reset()
         out = t.generate_argmax(1, 0, positions, forced=forced, stop_on_bos=False)
         assert len(out) == positions
+        last["tokens"] = out
         return t.last_timing()
+
+    def overwrite_state():
+        """The same positions from other tokens (untimed): the context keeps logits, x and the KV cache
+        across calls, and every warm-up run leaves the values the next step should compute, so without
+        this a step that skipped a kernel would still leave the expected values behind."""
+        t.reset()
+        other = (teacher_tokens(positions + 1, ck.vocab_size)[1:] + 1) % ck.vocab_size
+        t.generate_argmax(2, 0, positions, forced=other, stop_on_bos=False)
 
     host_lib, GenOptions, GenResult = load_host_twin()
     opt = GenOptions(0.0, 0.9, positions, 0, 0, 0, 0)
@@ -348,7 +390,9 @@ def run_workload(workload, args, rank, world, dist, sync, flush, clock_index):
     # ---- timed: K device-resident steps, each bracketed by barrier + synchronize, L2 flushed before
     step_s, dev_ms, launches = [], [], 0
     with ClockSampler(clock_index) as clocks:
-        for _ in range(args.steps):
+        for i in range(args.steps):
+            if args.dump_outputs and i == args.steps - 1:
+                overwrite_state()
             flush()
             sync()
             t0 = time.perf_counter()
@@ -357,6 +401,8 @@ def run_workload(workload, args, rank, world, dist, sync, flush, clock_index):
             step_s.append(time.perf_counter() - t0)
             dev_ms.append(ms)
             launches += k
+        outputs = (step_outputs(t, positions, last["tokens"], world == 1 and args.in_process <= 1)
+                   if args.dump_outputs and rank == 0 else None)
         # ---- e2e: same positions through l2b_forward with host buffers
         e2e_s, h2d, d2h = [], 0, 0
         for _ in range(max(1, min(args.steps, 5))):
@@ -430,7 +476,7 @@ def run_workload(workload, args, rank, world, dist, sync, flush, clock_index):
                        "note": "stories15M's 61 MB of weights stay in the 126 MB L2 after the first token"
                                if workload == "stories15M" else "weights exceed L2: HBM-served"},
         "kernels": kernels, "clocks": clocks.summary(), "data": data_desc,
-        "weights_bytes_per_token_per_gpu": int(wbytes),
+        "weights_bytes_per_token_per_gpu": int(wbytes), "outputs": outputs,
     }
     if world > 1 and forced is not None:
         out["parity"] = tp_parity(t, ck, workload, rank, device)
@@ -462,7 +508,15 @@ def main():
     ap.add_argument("--in-process", type=int, default=0, metavar="N",
                     help="ONE process drives N GPUs (l2b_create(.., n_gpus=N), what the Zig CLI's --gpus uses) "
                          "instead of one process per GPU; run without torchrun")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what each workload's last timed step computed "
+                         "(logits, x, sampled key/value cache; tokens, the forced input under teacher "
+                         "forcing) to DIR/<workload>_<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a sample whose length varies")
 
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -494,15 +548,19 @@ def main():
     workload = pick_workload(args)
     clock_index = int(os.environ.get("LOCAL_RANK", 0))
     main_res = run_workload(workload, args, rank, world, dist, sync, flush, clock_index)
+    outputs = {workload: main_res["outputs"]}
     also = {}
     if world == 1 and args.also != "none" and args.in_process <= 1:
         extra = ["stories15M", "stories110M"] if args.also == "auto" else [w for w in args.also.split(",") if w]
         for w in extra:
             if w != workload:
                 r = run_workload(w, args, rank, world, dist, sync, flush, clock_index)
+                outputs[w] = r["outputs"]
                 also[w] = {k: r[k] for k in ("value", "ms_per_step", "device_ms_per_step", "e2e", "roofline",
                                              "whole_step", "kernels", "positions", "data", "prefill") if k in r}
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         cpu = None
         if not args.no_cpu_baseline and world == 1 and args.in_process <= 1:
             cpu = cpu_port_run(workload, budget_s=12.0)

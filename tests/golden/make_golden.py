@@ -6,11 +6,14 @@ no Zig toolchain exists in this image, see oracle/llama2_oracle.h "Pinning statu
                              float mode; sha256 matches SURVEY.md Appendix B.
   stories15M_logits.npz      logits of selected positions along that stream (every 16th logit
                              + the top-32), oracle strict W=8.
+  stories15M_header.bin      the checkpoint's 28-byte header (its size is in the tokens file).
+  tokenizer.bin.xz           the shipped tokenizer.bin, xz-compressed.
 
-Run here (needs /root/reference or assets/stories15M.bin):  python tests/golden/make_golden.py
+Needs the real assets/stories15M.bin and assets/tokenizer.bin:  python tests/golden/make_golden.py
 """
 import hashlib
 import json
+import lzma
 import os
 import sys
 
@@ -20,13 +23,18 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 import oracle_lib as O  # noqa: E402
 
-CKPT = next(p for p in ("/root/reference/stories15M.bin",
-                        os.path.join(os.path.dirname(os.path.dirname(HERE)), "assets", "stories15M.bin"))
-            if os.path.exists(p))
+ASSETS = os.path.join(os.path.dirname(os.path.dirname(HERE)), "assets")
+CKPT = os.path.join(ASSETS, "stories15M.bin")
 POSITIONS = [0, 1, 2, 50, 98, 150, 220, 221]
 
 
 def main():
+    with open(CKPT, "rb") as f, open(os.path.join(HERE, "stories15M_header.bin"), "wb") as out:
+        out.write(f.read(28))
+    with open(os.path.join(ASSETS, "tokenizer.bin"), "rb") as f:
+        packed = lzma.compress(f.read(), preset=9 | lzma.PRESET_EXTREME)
+    with open(os.path.join(HERE, "tokenizer.bin.xz"), "wb") as out:
+        out.write(packed)
     streams = {}
     for kind in ("strict", "fast"):
         cfg, shared, data = O.read_checkpoint(CKPT, kind)

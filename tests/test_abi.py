@@ -1,6 +1,7 @@
 """CPU: the C-ABI library loads and exports every symbol include/llama2_b200.h declares;
 argument validation and the no-fallback rule hold without a GPU (no compute calls here)."""
 import ctypes as C
+import json
 import os
 import subprocess
 
@@ -78,10 +79,18 @@ def test_no_cpu_fallback_when_no_device(l2b):
         l2b.matmul(np.zeros(3, np.float32), np.ones(3, np.float32), np.ones(9, np.float32))
 
 
-def test_checkpoint_floats_matches_real_file(l2b, stories15m):
-    ck = l2b.read_checkpoint(stories15m)
+def test_checkpoint_floats_matches_real_file(l2b, tmp_path):
+    """stories15M.bin's own 28-byte header, padded with zeros to the real file's size (sparse)."""
+    golden = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    with open(os.path.join(golden, "stories15M_t0_tokens.json")) as f:
+        size = json.load(f)["checkpoint_bytes"]
+    path = tmp_path / "stories15M.bin"
+    with open(os.path.join(golden, "stories15M_header.bin"), "rb") as f, open(path, "wb") as out:
+        out.write(f.read())
+        out.truncate(size)
+    ck = l2b.read_checkpoint(str(path))
     assert ck.shape_tuple == (288, 768, 6, 6, 6, 32000, 256) and ck.shared_weights
-    assert l2b.checkpoint_floats(ck) == ck.data.size == (os.path.getsize(stories15m) - 28) // 4
+    assert l2b.checkpoint_floats(ck) == ck.data.size == (os.path.getsize(path) - 28) // 4
 
 
 def test_product_never_references_the_oracle():

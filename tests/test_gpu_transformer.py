@@ -22,6 +22,21 @@ def teacher_tokens(n, vocab):
     return [(1 + 7919 * p) % vocab for p in range(n)]      # SURVEY.md 8d
 
 
+def is_argmax_within_tol(idx, logits):
+    """idx is an argmax of `logits` up to REL_TOL: a near-tie may legitimately break either way when
+    the summation order differs (as test_stories110m_full_depth_full_context allows)."""
+    return float(logits[idx]) >= float(np.max(logits)) - REL_TOL * float(np.max(np.abs(logits)))
+
+
+def stories15m_synthetic(l2b):
+    """stories15M's shape with bench.py's synthetic weights (seed 15): the 61 MB checkpoint is not stored
+    in the repository, and these tests need a model of that shape, not its trained weights."""
+    from llama2_zig_b200.checkpoint import shape_checkpoint
+    ck = shape_checkpoint("stories15M")
+    ck.data = l2b.synth_checkpoint_host(ck, 15)
+    return ck
+
+
 def make_pair(l2b, oracle, shape, seed):
     from llama2_zig_b200.checkpoint import shape_checkpoint
     ck = shape_checkpoint(shape)
@@ -103,10 +118,10 @@ def test_stories15m_argmax_and_generate_paths(l2b, stories15m):
         assert out3.tolist() == gold["tokens"][:40]
 
 
-def test_rope_table_from_host_is_used(l2b, oracle, stories15m):
+def test_rope_table_from_host_is_used(l2b, oracle):
     """rope_cos/rope_sin passed through the ABI (host libm) give the same result as the
     library's own table here (same libm); a deliberately wrong table must change the logits."""
-    ck = l2b.read_checkpoint(stories15m, mmap=False)
+    ck = stories15m_synthetic(l2b)
     hs = ck.dim // ck.n_heads
     import ctypes as C
     lib = oracle.load("strict")
@@ -175,8 +190,8 @@ def test_long_context_attention_splits(l2b, oracle):
                 om.forward(tok, pos)
 
 
-def test_call_order_and_argument_errors(l2b, stories15m):
-    ck = l2b.read_checkpoint(stories15m, mmap=False)
+def test_call_order_and_argument_errors(l2b):
+    ck = stories15m_synthetic(l2b)
     with l2b.Transformer(ck) as t:
         with pytest.raises(l2b.L2BError) as e:
             t.forward(1, 5)                      # skips ahead of the KV cache
@@ -192,8 +207,8 @@ def test_call_order_and_argument_errors(l2b, stories15m):
         assert np.array_equal(a, b)
 
 
-def test_determinism_and_reset(l2b, stories15m):
-    ck = l2b.read_checkpoint(stories15m, mmap=False)
+def test_determinism_and_reset(l2b):
+    ck = stories15m_synthetic(l2b)
     with l2b.Transformer(ck) as t:
         run1 = [t.forward(tok, pos) for pos, tok in enumerate([1, 9038, 2501, 263, 931])]
         t.reset()
@@ -261,21 +276,20 @@ def test_llama2_7b_full_depth(l2b, oracle):
             assert np.array_equal(t2.forward(tok, pos), got[pos]), pos
 
 
-def test_forward_sample_matches_host_sampler_steps(l2b, oracle, stories15m):
+def test_forward_sample_matches_host_sampler_steps(l2b, oracle):
     """l2b_forward_sample: transformer() + logits/=T + softmax + top-p prefilter (:996, :1005-1012)
     against the oracle's logits pushed through the reference's own host-side steps."""
     import ctypes as C
     FP = C.POINTER(C.c_float)
-    ck = l2b.read_checkpoint(stories15m, mmap=False)
-    cfg, shared, data = oracle.read_checkpoint(stories15m)
-    om = oracle.OracleModel(cfg, data, shared, W=8, kind="strict")
+    ck, om = make_pair(l2b, oracle, "stories15M", 15)
     lib = oracle.load("strict")
     with l2b.Transformer(ck) as t:
         tok = 1
         for pos, (temp, top_p) in enumerate([(1.0, 0.9), (0.8, 0.9), (1.0, 0.0), (1.5, 0.5), (0.5, 1.0), (1.0, 0.95)]):
             probs, cand = t.forward_sample(tok, pos, temp, top_p)
-            want = om.forward(tok, pos)
-            nxt = int(np.argmax(want))
+            raw = om.forward(tok, pos)
+            nxt = int(np.argmax(raw))
+            want = raw.copy()
             if temp != 1.0:
                 want = (want / np.float32(temp)).astype(np.float32)
             ref64 = np.exp(want.astype(np.float64) - want.max())
@@ -284,12 +298,12 @@ def test_forward_sample_matches_host_sampler_steps(l2b, oracle, stories15m):
             # The bar is the exact softmax (1e-4, the north star's tolerance).  The reference itself sums the
             # 32000 exponentials sequentially in fp32 (:697-701): once the running sum has absorbed the
             # dominant term (~1.0), terms below its half-ulp (6e-8) are rounded away one by one, so on a sharp
-            # distribution (T = 0.5: p_max = 0.985, the other 31999 terms share 0.015) its normalisation is
-            # off by ~1e-3.  The device's tree sum does not reproduce that loss; against the restatement the
-            # bar is therefore 2e-3, and the argmax / candidate set are compared exactly below.
+            # distribution (p_max near 1, e.g. the trained stories15M at T = 0.5: 0.985) its normalisation is
+            # off by up to ~1e-3.  The device's tree sum does not reproduce that loss; against the restatement
+            # the bar is therefore 2e-3.  The argmax is compared up to a near-tie, the candidate set exactly.
             assert np.max(np.abs(probs - ref64)) <= 1e-4 * np.max(ref64)
             assert np.max(np.abs(probs - want)) <= 2e-3 * np.max(want)
-            assert int(np.argmax(probs)) == nxt
+            assert int(np.argmax(probs)) == nxt or is_argmax_within_tol(int(np.argmax(probs)), raw)
             if top_p in (0.0, 1.0):
                 assert cand is None
             else:
@@ -300,10 +314,10 @@ def test_forward_sample_matches_host_sampler_steps(l2b, oracle, stories15m):
             tok = nxt
 
 
-def test_logits_buffer_is_zero_copy_state_logits(l2b, stories15m):
+def test_logits_buffer_is_zero_copy_state_logits(l2b):
     """A host that adopts l2b_logits_buffer() as state.logits (src/main.zig:149) gets the same
     logits as one that passes its own buffer."""
-    ck = l2b.read_checkpoint(stories15m, mmap=False)
+    ck = stories15m_synthetic(l2b)
     with l2b.Transformer(ck) as t:
         buf = t.logits_buffer()
         for pos, tok in enumerate([1, 9038, 2501]):
@@ -311,23 +325,24 @@ def test_logits_buffer_is_zero_copy_state_logits(l2b, stories15m):
             t.forward_into(tok, pos, buf)
             assert np.array_equal(own, buf)
         ms, nbytes = t.load_stats()
-        assert nbytes == 60_816_028 - 28 - 4 * 2 * 256 * 24 and ms > 0      # freq_cis tables are not uploaded
+        assert nbytes == 60_816_028 - 28 - 4 * 2 * 256 * 24 and ms > 0      # stories15M.bin less header and freq_cis tables
 
 
-def test_prefill_equals_token_by_token(l2b, oracle, stories15m):
+def test_prefill_equals_token_by_token(l2b, oracle):
     """SURVEY 8f.2: l2b_prefill (all prompt positions on the device, classifier skipped where the
     reference discards the logits, src/main.zig:996-1000) leaves the same KV cache and returns the
     same logits as feeding the prompt through l2b_forward one token at a time — bit for bit."""
     with open(os.path.join(GOLDEN, "stories15M_t0_tokens.json")) as f:
         gold = json.load(f)["tokens"]
     prompt = [1] + gold[:23]                      # BOS + 23 story tokens
-    ck = l2b.read_checkpoint(stories15m, mmap=False)
+    ck, om = make_pair(l2b, oracle, "stories15M", 15)
     with l2b.Transformer(ck) as a, l2b.Transformer(ck) as b:
         for pos, tok in enumerate(prompt):
             want = a.forward(tok, pos)
+            ref = om.forward(tok, pos)
         got = b.prefill(prompt, 0)
         assert np.array_equal(got, want)
-        assert int(np.argmax(got)) == gold[23]
+        assert rel_err(got, ref) <= REL_TOL
         n = 6 * 256 * 288
         assert np.array_equal(a.state("key_cache")[:n], b.state("key_cache")[:n])
         assert np.array_equal(a.state("value_cache")[:n], b.state("value_cache")[:n])
@@ -336,9 +351,12 @@ def test_prefill_equals_token_by_token(l2b, oracle, stories15m):
         assert b.prefill(prompt + gold[23:40], 0, want_logits=False) is None
         for pos in range(len(prompt), len(prompt) + 17):
             a.forward(gold[pos - 1], pos)
+            om.forward(gold[pos - 1], pos)
         nxt_a = a.forward_argmax(gold[40], 41)
         nxt_b = b.forward_argmax(gold[40], 41)
-        assert nxt_a == nxt_b == gold[41]
+        ref = om.forward(gold[40], 41)
+        assert nxt_a == nxt_b
+        assert nxt_a == int(np.argmax(ref)) or is_argmax_within_tol(nxt_a, ref)
         with pytest.raises(l2b.L2BError):
             b.prefill([1] * 300, 0)               # runs past seq_len
 

@@ -2,12 +2,15 @@
 sampler behave like src/main.zig.  The tokenizer checks are the reference's own `bpe` test
 (src/main.zig:1152-1180) replayed on the shipped tokenizer.bin."""
 import ctypes as C
+import hashlib
+import lzma
 import os
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+TOKENIZER_SHA256 = "74f899535f8f99cdeac697474b697f3fa40467b8376dab7b6c4d8c753f28ae9f"
 
 
 @pytest.fixture(scope="module")
@@ -32,20 +35,21 @@ def host():
     return lib
 
 
-def tokenizer_path():
-    for p in (os.path.join(ROOT, "assets", "tokenizer.bin"), "/root/reference/tokenizer.bin"):
-        if os.path.exists(p):
-            return p
-    return None
+@pytest.fixture(scope="module")
+def tokenizer(tmp_path_factory):
+    """The reference's shipped tokenizer.bin, stored xz-compressed under tests/golden."""
+    with lzma.open(os.path.join(ROOT, "tests", "golden", "tokenizer.bin.xz")) as f:
+        data = f.read()
+    assert hashlib.sha256(data).hexdigest() == TOKENIZER_SHA256
+    path = tmp_path_factory.mktemp("tokenizer") / "tokenizer.bin"
+    path.write_bytes(data)
+    return str(path)
 
 
-def test_bpe(host):
+def test_bpe(host, tokenizer):
     """test "bpe", src/main.zig:1152-1180."""
-    path = tokenizer_path()
-    if path is None:
-        pytest.skip("tokenizer.bin not staged")
     tk = C.c_void_p()
-    assert host.l2h_tokenizer_load(path.encode(), 32000, C.byref(tk)) == 0
+    assert host.l2h_tokenizer_load(tokenizer.encode(), 32000, C.byref(tk)) == 0
     assert host.l2h_tokenizer_lookup(tk, "æ".encode(), 2) == 233
     n = C.c_int32()
     p = host.l2h_tokenizer_token(tk, 100, C.byref(n))
@@ -81,14 +85,11 @@ def test_sampler_helpers(host):
         assert host.l2h_sample_top_p(peaked.ctypes.data_as(FP), 4, 0.9, scratch) == 1
 
 
-def test_tokenizer_hash_lookup_equals_first_match_scan(host):
+def test_tokenizer_hash_lookup_equals_first_match_scan(host, tokenizer):
     """SURVEY 8f.4: the O(1) lookup must answer exactly like the reference's linear scan (:208-215):
     the FIRST id whose bytes match — the shipped vocabulary has 204 duplicated strings."""
-    path = tokenizer_path()
-    if path is None:
-        pytest.skip("tokenizer.bin not staged")
     tk = C.c_void_p()
-    assert host.l2h_tokenizer_load(path.encode(), 32000, C.byref(tk)) == 0
+    assert host.l2h_tokenizer_load(tokenizer.encode(), 32000, C.byref(tk)) == 0
     first, dups = {}, 0
     n = C.c_int32()
     for i in range(32000):
