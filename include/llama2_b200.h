@@ -14,7 +14,8 @@
  *     :534-540, become argument checks);
  *   - host pointers are borrowed for the duration of the call only;
  *   - one context = one decode stream on 1, 2, 4 or 8 GPUs; not thread-safe (the reference is
- *     single-threaded);
+ *     single-threaded); contexts that share one set of weights (l2b_create_stream) are driven
+ *     from one thread, like a single context;
  *   - there is NO CPU fallback: if no sm_100 device is usable the call fails with
  *     L2B_ERR_CUDA / L2B_ERR_NO_DEVICE.
  */
@@ -173,6 +174,41 @@ int32_t l2b_generate_argmax(l2b_ctx *ctx, int32_t token, int32_t pos, int32_t n_
  * l2b_forward bit for bit.                                                                 */
 int32_t l2b_prefill(l2b_ctx *ctx, const int32_t *tokens, int32_t n_tokens, int32_t pos0,
                     float *host_logits);
+
+/* ---- several decode streams over one copy of the weights ----------------------------- */
+
+#define L2B_MAX_BATCH 8
+
+/* A new decode stream over base's device weights: its own KV cache, run state, control block,
+ * pinned buffers and graphs; no weight upload (l2b_load_stats reports 0 bytes).  Weights are
+ * reference-counted: base may be destroyed before its streams.  Single-GPU contexts only (a
+ * sharded or in-process-group base => L2B_ERR_UNSUPPORTED).  A stream is an ordinary l2b_ctx:
+ * every existing call (forward, prefill, forward_sample, generate_argmax, reset, read_state...)
+ * works on it unchanged.                                                                   */
+int32_t l2b_create_stream(l2b_ctx **out, l2b_ctx *base);
+
+/* One transformer() step for each of n streams (distinct, over the same weights,
+ * 1 <= n <= L2B_MAX_BATCH): tokens[k] at pos[k] on streams[k]; host_logits is [n][vocab].  Per
+ * stream the result equals l2b_forward on that stream alone.  On bandwidth-bound shapes (today
+ * llama2-7B on one GPU) up to 4 streams share each pass over the weights; on every other shape the
+ * streams' own steps run in turn (same results, no speed-up).
+ * Errors: NULL pointers, n outside 1..L2B_MAX_BATCH, a stream listed twice, streams over different
+ * weights, token or pos out of range => L2B_ERR_INVALID_ARG; pos[k] beyond what streams[k] has
+ * appended => L2B_ERR_STATE.  l2b_last_timing(streams[0]) reports the device time and kernel
+ * launches of the call; every stream's appended length is updated, so single-stream calls continue
+ * any stream.  What l2b_read_state returns for x / xb / hb / q / logits of a stream after a batch
+ * call is unspecified (its KV cache rows are exact).                                        */
+int32_t l2b_forward_batch(l2b_ctx *const *streams, int32_t n, const int32_t *tokens,
+                          const int32_t *pos, float *host_logits);
+
+/* l2b_generate_argmax for n streams stepping together on the device, with no host round trip per
+ * step.  forced is [n][n_steps] (or NULL; -1 = free-running), out_next is [n][n_steps], n_done is
+ * [n].  Steps of stream k are clamped to seq_len - pos[k]; a stream that emits BOS with stop_on_bos
+ * stops (its KV cache and outputs stay as the single-stream loop would leave them) while the others
+ * continue.  Argument checks, timing and state as l2b_forward_batch.                        */
+int32_t l2b_generate_argmax_batch(l2b_ctx *const *streams, int32_t n, const int32_t *tokens,
+                                  const int32_t *pos, int32_t n_steps, const int32_t *forced,
+                                  int32_t stop_on_bos, int32_t *out_next, int32_t *n_done);
 
 /* ---- introspection ------------------------------------------------------------------- */
 

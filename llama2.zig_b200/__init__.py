@@ -30,12 +30,15 @@ from .binding import (  # noqa: F401
     fused_matmul,
     sample_prep,
     exported_symbols,
+    forward_batch,
+    generate_argmax_batch,
 )
 from .checkpoint import Checkpoint, read_checkpoint, MODEL_SHAPES  # noqa: F401
 
 __all__ = [
     "L2BError", "L2BConfig", "L2BShard", "Transformer", "checkpoint_floats", "comm_unique_id",
     "lib_path", "load_library", "matmul", "rmsnorm", "softmax", "synth_checkpoint_host",
-    "vector_weighted_sum_rows", "attention_head", "fused_matmul", "sample_prep", "exported_symbols", "Checkpoint",
+    "vector_weighted_sum_rows", "attention_head", "fused_matmul", "sample_prep", "exported_symbols", "forward_batch",
+    "generate_argmax_batch", "Checkpoint",
     "read_checkpoint", "MODEL_SHAPES",
 ]

@@ -80,6 +80,9 @@ def load_library():
     lib.l2b_create_synthetic.argtypes = [C.POINTER(vp), C.POINTER(L2BConfig), C.c_uint64,
                                          C.POINTER(L2BShard)]
     lib.l2b_create_synthetic_group.argtypes = [C.POINTER(vp), C.POINTER(L2BConfig), C.c_uint64, C.c_int32]
+    lib.l2b_create_stream.argtypes = [C.POINTER(vp), vp]
+    lib.l2b_forward_batch.argtypes = [C.POINTER(vp), C.c_int32, IP, IP, FP]
+    lib.l2b_generate_argmax_batch.argtypes = [C.POINTER(vp), C.c_int32, IP, IP, C.c_int32, IP, C.c_int32, IP, IP]
     lib.l2b_destroy.argtypes = [vp]
     lib.l2b_destroy.restype = None
     lib.l2b_reset.argtypes = [vp]
@@ -171,13 +174,17 @@ class Transformer:
     """
 
     def __init__(self, ck, synthetic_seed=None, rank=0, world_size=1, device=0, comm_id=None,
-                 rope_cos=None, rope_sin=None, n_gpus=1):
+                 rope_cos=None, rope_sin=None, n_gpus=1, _stream_of=None):
         """n_gpus > 1: ONE process drives n_gpus GPUs (l2b_create(.., n_gpus)); rank/world_size:
         one process per GPU (l2b_create_sharded)."""
         self.lib = load_library()
         self.ck = ck
         self.cfg = make_config(ck)
         self.h = C.c_void_p()
+        if _stream_of is not None:           # new_stream(): l2b_create_stream over another context's weights
+            _check(self.lib.l2b_create_stream(C.byref(self.h), _stream_of.h), _stream_of.h)
+            self._logits = np.empty(ck.vocab_size, dtype=np.float32)
+            return
         shard = None
         assert n_gpus == 1 or world_size == 1
         if world_size > 1 or device != 0 or rank != 0:
@@ -231,6 +238,11 @@ class Transformer:
 
     def reset(self):
         _check(self.lib.l2b_reset(self.h), self.h)
+
+    def new_stream(self):
+        """Another decode stream over this context's device weights (l2b_create_stream): its own KV
+        cache and run state, no upload.  The weights live as long as any context that uses them."""
+        return Transformer(self.ck, _stream_of=self)
 
     # -- the hot path
     def forward(self, token, pos):
@@ -325,6 +337,55 @@ class Transformer:
         kv = C.c_uint64()
         _check(self.lib.l2b_step_bytes(self.h, int(pos), C.byref(w), C.byref(kv)), self.h)
         return w.value, kv.value
+
+
+# ---- several decode streams over one copy of the weights -------------------------------------
+
+def _batch_args(streams, tokens, positions):
+    n = len(streams)
+    hs = (C.c_void_p * max(n, 1))(*[s.h.value for s in streams])
+    toks = np.ascontiguousarray(tokens, dtype=np.int32)
+    pos = np.ascontiguousarray(positions, dtype=np.int32)
+    if toks.size != n or pos.size != n:
+        raise ValueError("one token and one position per stream")
+    return n, hs, toks, pos
+
+
+def _batch_check(rc, streams):
+    _check(rc, streams[0].h if streams else None)
+
+
+def forward_batch(streams, tokens, positions):
+    """One transformer() step on each stream (l2b_forward_batch): tokens[k] at positions[k] on
+    streams[k], all Transformers over the same weights.  Returns (n, vocab) logits."""
+    lib = load_library()
+    n, hs, toks, pos = _batch_args(streams, tokens, positions)
+    vocab = streams[0].ck.vocab_size if streams else 1
+    out = np.empty((max(n, 1), vocab), dtype=np.float32)
+    rc = lib.l2b_forward_batch(hs, n, toks.ctypes.data_as(IP), pos.ctypes.data_as(IP), out.ctypes.data_as(FP))
+    _batch_check(rc, streams)
+    return out[:n]
+
+
+def generate_argmax_batch(streams, tokens, positions, n_steps, forced=None, stop_on_bos=True):
+    """Transformer.generate_argmax for every stream at once on the device
+    (l2b_generate_argmax_batch).  forced: (n, n_steps) ints, -1 = free-running, or None.  Returns a
+    list with each stream's chosen tokens."""
+    lib = load_library()
+    n, hs, toks, pos = _batch_args(streams, tokens, positions)
+    width = max(int(n_steps), 1)
+    out = np.full((max(n, 1), width), -1, dtype=np.int32)
+    done = np.zeros(max(n, 1), dtype=np.int32)
+    fp = None
+    if forced is not None:
+        forced = np.ascontiguousarray(forced, dtype=np.int32).reshape(n, -1)
+        if forced.shape[1] != n_steps:
+            raise ValueError("forced must be (n, n_steps)")
+        fp = forced.ctypes.data_as(IP)
+    rc = lib.l2b_generate_argmax_batch(hs, n, toks.ctypes.data_as(IP), pos.ctypes.data_as(IP), int(n_steps), fp,
+                                       1 if stop_on_bos else 0, out.ctypes.data_as(IP), done.ctypes.data_as(IP))
+    _batch_check(rc, streams)
+    return [out[k, :done[k]].copy() for k in range(n)]
 
 
 # ---- reference-named single ops on host buffers (device = cuda:0) ---------------------------

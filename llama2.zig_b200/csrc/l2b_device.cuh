@@ -1101,6 +1101,18 @@ __global__ void __launch_bounds__(NT) gemv_scalar_kernel(float *out, const float
 // by the last CTA of the head to arrive (threadfence + counter), in fixed split order, so the
 // result is deterministic.
 // ---------------------------------------------------------------------------------------
+// One activation vector of a batched pass (prompt prefill, or decode streams that share one copy of
+// the weights): its own token, position and KV cache.  Prefill fills consecutive positions of one
+// cache; batched decode has one entry per stream.  Device memory, so a step reads it the way a
+// single-stream step reads ctl, and advance_batch_kernel moves it on without the host.
+struct BatchVec {
+    int token, pos;
+    int done;              // this vector's generation ended: every later kernel skips it (no KV append)
+    int step, limit;       // generate loop: steps taken, steps allowed
+    int pad;
+    float *kc, *vc;        // this vector's (n_layers, seq_len, kv_dim) key / value caches
+};
+
 struct AttnParams {
     const int *ctl;
     const float *q;        // (n_heads * head_size)
@@ -1112,9 +1124,12 @@ struct AttnParams {
     unsigned int *counters;  // (n_heads), zero between launches
     int head_size, kv_dim, kv_mul, nsplit, min_chunk;
     unsigned long long *trace;
-    // batched prompt prefill: gridDim.z positions at once; query z sits at position pos_base + z and
-    // uses q / xb / partial buffers offset by z (pos_base < 0: single position from the control block)
-    int pos_base, q_stride;
+    // batched passes: gridDim.z queries at once; query z takes its position, cache (vec[z].kc/vc +
+    // kv_off) and done flag from vec[z] and uses q / xb / partial buffers offset by z (vec == nullptr:
+    // single position from the control block, cache kcache / vcache)
+    const BatchVec *vec;
+    size_t kv_off;
+    int q_stride;
     int seq_len;           // rows of the cache (bounds the speculative first pass; 0 = no speculation)
 };
 
@@ -1315,7 +1330,8 @@ __global__ void __launch_bounds__(NT) attention_flash_kernel(const AttnParams p)
     const float *qz = p.q + (size_t)z * p.q_stride;
     const size_t hoff = (size_t)(h / p.kv_mul) * hs;          // :369, :382
     const float4 *q4 = reinterpret_cast<const float4 *>(qz + (size_t)h * hs);
-    const float *kb = p.kcache + hoff, *vb = p.vcache + hoff;
+    const float *kb = (p.vec ? p.vec[z].kc + p.kv_off : p.kcache) + hoff;
+    const float *vb = (p.vec ? p.vec[z].vc + p.kv_off : p.vcache) + hoff;
 
     // Everything whose ADDRESS does not depend on the position is requested before the position is
     // read from the control block: q, and (timeline split 0) the cache rows of this lane's first pass —
@@ -1343,8 +1359,8 @@ __global__ void __launch_bounds__(NT) attention_flash_kernel(const AttnParams p)
         }
     }
 
-    if (p.ctl[CTL_DONE]) return;
-    const int T = (p.pos_base >= 0 ? p.pos_base + z : p.ctl[CTL_POS]) + 1;
+    if (p.vec ? p.vec[z].done : p.ctl[CTL_DONE]) return;
+    const int T = (p.vec ? p.vec[z].pos : p.ctl[CTL_POS]) + 1;
     int chunk = (T + p.nsplit - 1) / p.nsplit;
     if (chunk < p.min_chunk) chunk = p.min_chunk;
     const int active = (T + chunk - 1) / chunk;
@@ -1683,6 +1699,33 @@ __global__ void advance_kernel(const AdvanceParams p) {
     ctl[CTL_TOKEN] = next;
     ctl[CTL_POS] = ctl[CTL_POS] + 1;
     ctl[CTL_STEP] = step + 1;
+}
+
+// advance_kernel for n decode streams stepping together (thread k = stream k): the forced token or
+// the stream's own argmax (amax[k], packed by the classifier's EPI_ARGMAX epilogue), recorded at
+// out_next[k * stride + step].  A stream that emits BOS with stop-on-BOS, or has taken its `limit`
+// steps, is marked done; every later kernel of the loop skips it.
+__global__ void advance_batch_kernel(BatchVec *vec, int n, unsigned long long *amax, const int *forced,
+                                     int *out_next, int *n_done, int stride, int stop_on_bos) {
+    pdl_wait();
+    const int k = threadIdx.x;
+    if (k >= n) return;
+    BatchVec &v = vec[k];
+    if (v.done) return;
+    const unsigned long long key = amax[k];
+    amax[k] = 0ull;
+    const int step = v.step;
+    int next = (int)(0xFFFFFFFFu - (unsigned int)(key & 0xFFFFFFFFull));
+    if (forced && forced[k * stride + step] >= 0) next = forced[k * stride + step];
+    out_next[k * stride + step] = next;
+    n_done[k] = step + 1;
+    if ((stop_on_bos && next == 1) || step + 1 >= v.limit) {   // :1017-1019
+        v.done = 1;
+        return;
+    }
+    v.token = next;
+    v.pos = v.pos + 1;
+    v.step = step + 1;
 }
 
 // Tensor parallel logits: every rank's classifier sent its vocab slice as LL units (EPI_XCHG with

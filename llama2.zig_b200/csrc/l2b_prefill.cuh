@@ -1,5 +1,7 @@
-// l2b_prefill.cuh — batched prompt prefill (SURVEY 8f.2): NB consecutive prompt positions share one
-// pass over the weights.
+// l2b_prefill.cuh — batched passes over the weights: NB activation vectors share one pass.  They are
+// consecutive positions of one prompt (prefill, SURVEY 8f.2) or one token of each of NB decode
+// streams over the same weights (l2b_forward_batch / l2b_generate_argmax_batch); each vector takes
+// its token, position and KV cache from a BatchVec table in device memory.
 //
 // The reference feeds prompt tokens through transformer() one at a time (src/main.zig:996-1000) and
 // streams every weight once per token.  For bandwidth-bound shapes (llama2-7B) the same streaming
@@ -18,22 +20,23 @@ namespace l2b {
 constexpr int PF_MAXB = 4;
 
 struct PrefillParams {
-    // ---- input vectors: NB contiguous vectors of n floats, or (layer 0) embedding rows of tokens[b]
+    // ---- input vectors: NB contiguous vectors of n floats, or (layer 0) embedding rows of vec[b].token
     const float *x_in;
     const float *emb;
-    const int *tokens;      // device array: the chunk's tokens
+    const BatchVec *vec;    // device table: the pass's vectors (token, position, KV cache, done)
     const float *gamma;     // rmsnorm gain => fused rmsnorm of every vector
     float *x_out;           // layer 0: CTA 0 writes the NB embedding rows here (the residual-stream batch)
     int n, nb;              // columns; positions in this chunk (<= NB)
     // ---- matrices
     const float *w0, *w1, *w2;
     int rows0, rows1, rows2, total_rows;
-    // ---- outputs: EPI_QKV: q batch [nb][rows0]; EPI_SILU: hb batch [nb][rows0]; EPI_RESID: x batch [nb][total_rows]
+    // ---- outputs: EPI_QKV: q batch [nb][rows0]; EPI_SILU: hb batch [nb][rows0]; EPI_RESID: x batch
+    // [nb][total_rows]; EPI_STORE / EPI_ARGMAX: logits batch [nb][total_rows]
     float *out0;
-    float *kcache, *vcache;             // this layer's (seq_len, kv_dim)
+    unsigned long long *amax;           // EPI_ARGMAX: packed argmax key of vector b at amax[b]
+    size_t kv_off;                      // EPI_QKV: this layer's offset in vec[b].kc / vc ((seq_len, kv_dim) per layer)
     const float *rope_cos, *rope_sin;   // (seq_len, head_size/2)
     int head_size, kv_dim;
-    int pos0;               // position of the chunk's first token
     int nstage;
 };
 
@@ -85,7 +88,7 @@ __global__ void __launch_bounds__(TMA_THREADS, 1) prefill_gemm_kernel(const Pref
     __shared__ uint64_t full[TMA_MAX_STAGES], empty[TMA_MAX_STAGES], xbar, tile_full[2], tile_free[2];
     __shared__ float scratch[NB][NWARP + 2];
     __shared__ float red[2][NWARP][GEMV8_R][NB];
-    __shared__ float rope_s[NB][2][128];                               // cos/sin rows of pos0 .. pos0+NB-1
+    __shared__ float rope_s[NB][2][128];                               // cos/sin rows of the vectors' positions
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int n4 = p.n >> 2;
@@ -153,19 +156,21 @@ __global__ void __launch_bounds__(TMA_THREADS, 1) prefill_gemm_kernel(const Pref
             const uint32_t bytes = (uint32_t)p.n * 4u;
             mbar_expect_tx(&xbar, bytes * (uint32_t)p.nb);
             if (p.emb) {
-                for (int b = 0; b < p.nb; ++b)                          // x[b] = token_embedding_table[tokens[b]], :295-296
-                    tma_load_1d(xs + (size_t)b * p.n, p.emb + (size_t)p.tokens[b] * p.n, bytes, &xbar);
+                for (int b = 0; b < p.nb; ++b)                          // x[b] = token_embedding_table[token], :295-296
+                    tma_load_1d(xs + (size_t)b * p.n, p.emb + (size_t)p.vec[b].token * p.n, bytes, &xbar);
             } else {
                 tma_load_1d(xs, p.x_in, bytes * (uint32_t)p.nb, &xbar);
             }
         }
-        if (EPI == EPI_QKV && tid >= NT + 32) {                        // epilogue warp: RoPE rows of the chunk's positions
+        if (EPI == EPI_QKV && tid >= NT + 32) {                        // epilogue warp: RoPE rows of the vectors' positions
             const int half = p.head_size >> 1;
-            for (int b = 0; b < p.nb; ++b)
+            for (int b = 0; b < p.nb; ++b) {
+                const int pos = p.vec[b].pos;
                 for (int i = lane; i < half; i += 32) {
-                    rope_s[b][0][i] = __ldg(p.rope_cos + (size_t)(p.pos0 + b) * half + i);
-                    rope_s[b][1][i] = __ldg(p.rope_sin + (size_t)(p.pos0 + b) * half + i);
+                    rope_s[b][0][i] = __ldg(p.rope_cos + (size_t)pos * half + i);
+                    rope_s[b][1][i] = __ldg(p.rope_sin + (size_t)pos * half + i);
                 }
+            }
         }
         mbar_wait(&xbar, 0);
         if (p.gamma || p.x_out) {
@@ -222,8 +227,13 @@ __global__ void __launch_bounds__(TMA_THREADS, 1) prefill_gemm_kernel(const Pref
 
     if (warp == NWARP + 1) {
         // ---- epilogue warp: lane = b * 4 + pair handles (row pair, position b) of each tile
+        // (a vector whose generation has ended writes nothing: no KV append, no residual update)
         const int eb = lane >> 2, ep = lane & 3;
-        const bool active = lane < 4 * NB && eb < p.nb;
+        const bool active = lane < 4 * NB && eb < p.nb && !p.vec[eb].done;
+        int pos = 0;
+        float *kc = nullptr, *vc = nullptr;
+        if (EPI == EPI_QKV && active) { pos = p.vec[eb].pos; kc = p.vec[eb].kc + p.kv_off; vc = p.vec[eb].vc + p.kv_off; }
+        unsigned long long best = 0ull;
         for (int t = 0; t < ntiles; ++t) {
             const int par = t & 1, use = t >> 1;
             mbar_wait(&tile_full[par], use & 1);
@@ -239,7 +249,6 @@ __global__ void __launch_bounds__(TMA_THREADS, 1) prefill_gemm_kernel(const Pref
             if (lane == 0) mbar_arrive(&tile_free[par]);
             const int vp = r0 + t * GEMV8_R + 2 * ep;
             if (!active || vp >= r1) continue;
-            const int pos = p.pos0 + eb;
             if (EPI == EPI_QKV) {
                 if (vp < p.rows0 + p.rows1) {
                     const bool is_q = vp < p.rows0;
@@ -248,15 +257,27 @@ __global__ void __launch_bounds__(TMA_THREADS, 1) prefill_gemm_kernel(const Pref
                     const float fcr = rope_s[eb][0][pr], fci = rope_s[eb][1][pr];
                     const float q0 = __fsub_rn(__fmul_rn(s0, fcr), __fmul_rn(s1, fci));      // :348
                     const float q1 = __fadd_rn(__fmul_rn(s0, fci), __fmul_rn(s1, fcr));      // :349
-                    float *dst = is_q ? p.out0 + (size_t)eb * p.rows0 + i : p.kcache + (size_t)pos * p.kv_dim + i;   // :355,:357
+                    float *dst = is_q ? p.out0 + (size_t)eb * p.rows0 + i : kc + (size_t)pos * p.kv_dim + i;   // :355,:357
                     *reinterpret_cast<float2 *>(dst) = make_float2(q0, q1);
                 } else {
                     const int i = vp - p.rows0 - p.rows1;
-                    *reinterpret_cast<float2 *>(p.vcache + (size_t)pos * p.kv_dim + i) = make_float2(s0, s1);   // :356,:358
+                    *reinterpret_cast<float2 *>(vc + (size_t)pos * p.kv_dim + i) = make_float2(s0, s1);   // :356,:358
                 }
             } else if (EPI == EPI_SILU) {
                 const float sg = __fmul_rn(s0, __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-s0))));   // :412
                 p.out0[(size_t)eb * p.rows0 + (vp >> 1)] = __fmul_rn(sg, s1);                  // :416
+            } else if (EPI == EPI_STORE || EPI == EPI_ARGMAX) {   // logits row b (:429)
+                float *dst = p.out0 + (size_t)eb * p.total_rows + vp;
+                dst[0] = s0;
+                if (vp + 1 < p.total_rows) dst[1] = s1;
+                if (EPI == EPI_ARGMAX) {   // first maximum wins (:715-726), as gemv_epilogue_pair
+                    const unsigned long long k0 = argmax_key(s0, vp);
+                    best = k0 > best ? k0 : best;
+                    if (vp + 1 < p.total_rows) {
+                        const unsigned long long k1 = argmax_key(s1, vp + 1);
+                        best = k1 > best ? k1 : best;
+                    }
+                }
             } else {   // EPI_RESID: x[b][row] += acc (:395, :422)
                 float *dst = p.out0 + (size_t)eb * p.total_rows + vp;
                 if (vp + 1 < p.total_rows) {
@@ -266,6 +287,11 @@ __global__ void __launch_bounds__(TMA_THREADS, 1) prefill_gemm_kernel(const Pref
                     dst[0] += s0;
                 }
             }
+        }
+        if (EPI == EPI_ARGMAX) {   // the 4 lanes of vector b, then one 64-bit atomicMax per CTA and vector
+            best = max(best, __shfl_xor_sync(0xffffffffu, best, 1));
+            best = max(best, __shfl_xor_sync(0xffffffffu, best, 2));
+            if (active && ep == 0 && best) atomicMax(p.amax + eb, best);
         }
         return;
     }

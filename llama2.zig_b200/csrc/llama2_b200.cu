@@ -16,6 +16,7 @@
 #include <string.h>
 
 #include <chrono>
+#include <memory>
 #include <set>
 #include <string>
 #include <vector>
@@ -87,6 +88,33 @@ enum StepMode { MODE_LOGITS = 0, MODE_ARGMAX = 1, MODE_SAMPLE = 2, MODE_NOCLS = 
 enum GraphId { G_LOGITS = 0, G_ARGMAX_ONE = 1, G_ARGMAX_LOOP = 2, G_SAMPLE = 3, G_PREFILL_LOOP = 4, G_COUNT = 5 };
 constexpr int kCandCap = 8192;               // top-p candidates returned per step (more => host filters itself)
 
+// Device weights (Weights, src/main.zig:53-71) of one single-GPU context, shared by every decode stream
+// created over them (l2b_create_stream) and freed with the last context that uses them.  The scratch
+// of batched passes (prefill chunks, batched decode steps) lives here too: contexts over one set of
+// weights are driven from one thread and every call synchronises before it returns.
+struct WeightStore {
+    int device = 0;
+    std::vector<void *> owned;               // weight tensors and batch scratch (device)
+    std::vector<void *> pinned;              // batch scratch (pinned host)
+    bool batch_ready = false;
+    // [L2B_MAX_BATCH] vectors of dim | q | q | hidden | vocab floats
+    float *x = nullptr, *q = nullptr, *xb = nullptr, *hb = nullptr, *logits = nullptr;
+    float *part_o = nullptr, *part_ml = nullptr; // attention partials per vector
+    unsigned int *counters = nullptr;
+    unsigned long long *amax = nullptr;      // [L2B_MAX_BATCH] packed argmax keys
+    BatchVec *vec = nullptr;                 // [max(seq_len, L2B_MAX_BATCH)] per-vector table
+    int *forced = nullptr, *out = nullptr;   // [L2B_MAX_BATCH][seq_len]
+    int *n_done = nullptr;                   // [L2B_MAX_BATCH]
+    BatchVec *h_vec = nullptr;               // pinned mirrors
+    float *h_logits = nullptr;               // [L2B_MAX_BATCH][vocab]
+    int *h_ints = nullptr;                   // [L2B_MAX_BATCH][seq_len] tokens, then [L2B_MAX_BATCH] step counts
+    ~WeightStore() {
+        cudaSetDevice(device);
+        for (void *p : owned) cudaFree(p);
+        for (void *p : pinned) cudaFreeHost(p);
+    }
+};
+
 struct l2b_ctx {
     l2b_config cfg{};
     int rank = 0, world = 1, device = 0, num_sms = 0;
@@ -97,7 +125,8 @@ struct l2b_ctx {
     int dim = 0, hidden = 0, head_size = 0, kv_mul = 0;
     int q_dim = 0, kv_dim = 0;              // global
     int q_loc = 0, kv_loc = 0, hid_loc = 0, heads_loc = 0, vocab_loc = 0;
-    // device weights (Weights, src/main.zig:53-71), this rank's slices
+    // device weights (Weights, src/main.zig:53-71), this rank's slices, owned by `weights`
+    std::shared_ptr<WeightStore> weights;
     float *emb = nullptr, *rms_att = nullptr, *rms_ffn = nullptr, *rms_final = nullptr;
     float *wq = nullptr, *wk = nullptr, *wv = nullptr, *wo = nullptr;
     float *w1 = nullptr, *w2 = nullptr, *w3 = nullptr, *wcls = nullptr;
@@ -107,11 +136,8 @@ struct l2b_ctx {
     float *final_X = nullptr;                // which of the two holds x after a step
     float *attn_parts = nullptr;             // small-model fusion: (n_heads, dim) partial vectors of attention + wo
     bool fuse_attn = false;
-    // batched prompt prefill (l2b_prefill, bandwidth-bound shapes): PF_MAXB positions per weight pass
-    float *pf_x = nullptr, *pf_q = nullptr, *pf_xb = nullptr, *pf_hb = nullptr;   // [PF_MAXB][dim | q | q | hidden]
-    float *pf_part_o = nullptr, *pf_part_ml = nullptr;
-    unsigned int *pf_counters = nullptr;
-    int *pf_tokens = nullptr;
+    // batched passes (l2b_prefill, l2b_forward_batch, l2b_generate_argmax_batch) on bandwidth-bound
+    // shapes: PF_MAXB vectors per pass over the weights, scratch in `weights`
     bool pf_ready = false, pf_ok = false;
     int attn_R = 1;                          // CTAs per head cluster of attn_wo_kernel
     float *delta = nullptr;                  // L2B_TP=nccl baseline only: partial rows before the NCCL all-reduce
@@ -619,7 +645,7 @@ int launch_attention(l2b_ctx *ctx, int layer, cudaStream_t st) {
     a.kv_mul = ctx->kv_mul;
     a.nsplit = ctx->nsplit;
     a.min_chunk = ctx->min_chunk;
-    a.pos_base = -1;
+    a.vec = nullptr;                 // single position from the control block
     a.seq_len = ctx->cfg.seq_len;
     a.trace = trace_slot(ctx);
     size_t smem = ctx->attn_smem;
@@ -963,21 +989,19 @@ int preload_kernels(l2b_ctx *ctx) {
     size_t smem = 0;
     L2B_CUDA(ctx, cudaFuncGetAttributes(&fa, (const void *)pick_attention(ctx->head_size, true, &smem)));
     if (pick_attn_wo(ctx->head_size, &smem)) L2B_CUDA(ctx, cudaFuncGetAttributes(&fa, (const void *)pick_attn_wo(ctx->head_size, &smem)));
-    const void *others[] = {(const void *)attention_kernel, (const void *)advance_kernel, (const void *)gather_logits_kernel,
+    const void *others[] = {(const void *)attention_kernel, (const void *)advance_kernel, (const void *)advance_batch_kernel,
+                            (const void *)gather_logits_kernel,
                             (const void *)resid_add_kernel, (const void *)sample_prep_kernel, (const void *)synth_fill_kernel};
     for (const void *f : others) L2B_CUDA(ctx, cudaFuncGetAttributes(&fa, f));
     return L2B_OK;
 }
 
 // ---- creation, stage 1: weights + run state of one rank (no peer is touched) ------------------
-int create_rank(l2b_ctx *ctx, const l2b_config *cfg, const Source &src, const float *rope_cos,
-                const float *rope_sin, int rank, int world, int device) {
-    cudaDeviceProp prop{};
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) { ctx->err = "cudaGetDeviceProperties failed"; g_create_error = ctx->err; return L2B_ERR_CUDA; }
-    if (prop.major != 10) { ctx->err = "device is not compute capability 10.x (built for sm_100a only)"; g_create_error = ctx->err; return L2B_ERR_NO_DEVICE; }
+// shape of one rank's shard, and the device objects every context needs
+int open_rank(l2b_ctx *ctx, const l2b_config *cfg, int rank, int world, int device, int num_sms) {
     ctx->cfg = *cfg;
     ctx->rank = rank; ctx->world = world; ctx->device = device;
-    ctx->num_sms = prop.multiProcessorCount;
+    ctx->num_sms = num_sms;
     ctx->dim = cfg->dim; ctx->hidden = cfg->hidden_dim;
     ctx->head_size = cfg->dim / cfg->n_heads;
     ctx->kv_mul = cfg->n_heads / cfg->n_kv_heads;
@@ -993,6 +1017,17 @@ int create_rank(l2b_ctx *ctx, const l2b_config *cfg, const Source &src, const fl
     L2B_TRY(cuda_try(ctx, cudaEventCreate(&ctx->ev0), "cudaEventCreate"));
     L2B_TRY(cuda_try(ctx, cudaEventCreate(&ctx->ev1), "cudaEventCreate"));
     L2B_TRY(preload_kernels(ctx));
+    return L2B_OK;
+}
+
+int init_run_state(l2b_ctx *ctx, const float *rope_cos, const float *rope_sin, const l2b_ctx *rope_from);
+
+int create_rank(l2b_ctx *ctx, const l2b_config *cfg, const Source &src, const float *rope_cos,
+                const float *rope_sin, int rank, int world, int device) {
+    cudaDeviceProp prop{};
+    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) { ctx->err = "cudaGetDeviceProperties failed"; g_create_error = ctx->err; return L2B_ERR_CUDA; }
+    if (prop.major != 10) { ctx->err = "device is not compute capability 10.x (built for sm_100a only)"; g_create_error = ctx->err; return L2B_ERR_NO_DEVICE; }
+    L2B_TRY(open_rank(ctx, cfg, rank, world, device, prop.multiProcessorCount));
 
     const uint64_t dim = cfg->dim, hid = cfg->hidden_dim, L = cfg->n_layers, V = cfg->vocab_size, S = cfg->seq_len;
     const uint64_t hs = ctx->head_size, kvd = ctx->kv_dim;
@@ -1037,8 +1072,20 @@ int create_rank(l2b_ctx *ctx, const l2b_config *cfg, const Source &src, const fl
         if (ctx->stage[i]) { cudaFreeHost(ctx->stage[i]); ctx->stage[i] = nullptr; }
         if (ctx->stage_ev[i]) { cudaEventDestroy(ctx->stage_ev[i]); ctx->stage_ev[i] = nullptr; }
     }
+    // everything allocated so far is a weight tensor: it moves to the store that streams share
+    ctx->weights = std::make_shared<WeightStore>();
+    ctx->weights->device = device;
+    ctx->weights->owned.swap(ctx->owned);
+    return init_run_state(ctx, rope_cos, rope_sin, nullptr);
+}
 
-    // ---- run state
+// ---- run state of one context (RunState.init, :137-154): its KV cache, buffers, graphs' inputs.
+// rope_from != nullptr: copy that context's RoPE table (a stream over its weights)
+int init_run_state(l2b_ctx *ctx, const float *rope_cos, const float *rope_sin, const l2b_ctx *rope_from) {
+    const l2b_config *cfg = &ctx->cfg;
+    const int world = ctx->world, rank = ctx->rank;
+    const uint64_t dim = cfg->dim, L = cfg->n_layers, V = cfg->vocab_size, S = cfg->seq_len;
+    const uint64_t hs = ctx->head_size;
     L2B_TRY(dev_alloc(ctx, &ctx->X, dim));
     L2B_TRY(dev_alloc(ctx, &ctx->Xalt, dim));
     {
@@ -1106,7 +1153,10 @@ int create_rank(l2b_ctx *ctx, const l2b_config *cfg, const Source &src, const fl
     // ---- RoPE table (:338-342); the host's own libm values when the caller passes them
     {
         std::vector<float> hc(S * hs / 2), hsn(S * hs / 2);
-        if (rope_cos && rope_sin) {
+        if (rope_from) {
+            L2B_TRY(cuda_try(ctx, cudaMemcpy(hc.data(), rope_from->rope_cos, hc.size() * sizeof(float), cudaMemcpyDeviceToHost), "rope copy"));
+            L2B_TRY(cuda_try(ctx, cudaMemcpy(hsn.data(), rope_from->rope_sin, hsn.size() * sizeof(float), cudaMemcpyDeviceToHost), "rope copy"));
+        } else if (rope_cos && rope_sin) {
             memcpy(hc.data(), rope_cos, hc.size() * sizeof(float));
             memcpy(hsn.data(), rope_sin, hsn.size() * sizeof(float));
         } else {
@@ -1580,27 +1630,60 @@ int32_t l2b_forward_sample(l2b_ctx *ctx, int32_t token, int32_t pos, float tempe
 
 }  // extern "C" (templates below)
 
-// ---- batched prompt prefill (csrc/l2b_prefill.cuh) --------------------------------------------
+// ---- batched passes over the weights (csrc/l2b_prefill.cuh) ------------------------------------
 typedef void (*pf_fn)(const PrefillParams);
 template <int NB>
 pf_fn pf_pick(int epi) {
     switch (epi) {
     case EPI_QKV: return prefill_gemm_kernel<EPI_QKV, NB>;
     case EPI_SILU: return prefill_gemm_kernel<EPI_SILU, NB>;
+    case EPI_STORE: return prefill_gemm_kernel<EPI_STORE, NB>;
+    case EPI_ARGMAX: return prefill_gemm_kernel<EPI_ARGMAX, NB>;
     default: return prefill_gemm_kernel<EPI_RESID, NB>;
     }
 }
 constexpr size_t kPfSmemBudget = 227 * 1024 - 8192;   // the prefill kernels keep ~6.5 KB of static shared memory
 
-// can this context prefill PF_MAXB positions per weight pass?  Single GPU, flash attention, and all
-// four per-layer GEMVs bandwidth-bound shapes of the TMA-ring kernel; otherwise l2b_prefill runs the
-// positions one by one on the device (same results, weights streamed once per position).
+// scratch of the batched passes, once per set of weights (every context over them uses it in turn)
+static int alloc_batch_scratch(l2b_ctx *ctx, WeightStore &w) {
+    const size_t B = L2B_MAX_BATCH, S = ctx->cfg.seq_len, V = ctx->cfg.vocab_size;
+    const size_t nvec = S > B ? S : B;
+    int rc;
+    if ((rc = dev_alloc(ctx, &w.x, B * ctx->dim))) return rc;
+    if ((rc = dev_alloc(ctx, &w.q, B * ctx->q_loc))) return rc;
+    if ((rc = dev_alloc(ctx, &w.xb, B * ctx->q_loc))) return rc;
+    if ((rc = dev_alloc(ctx, &w.hb, B * ctx->hid_loc))) return rc;
+    if ((rc = dev_alloc(ctx, &w.logits, B * V))) return rc;
+    if ((rc = dev_alloc(ctx, &w.part_o, B * ctx->heads_loc * ctx->nsplit * ctx->head_size))) return rc;
+    if ((rc = dev_alloc(ctx, &w.part_ml, B * ctx->heads_loc * ctx->nsplit * 2))) return rc;
+    if ((rc = dev_alloc(ctx, &w.counters, B * ctx->heads_loc))) return rc;
+    if ((rc = dev_alloc(ctx, &w.amax, B))) return rc;
+    if ((rc = dev_alloc(ctx, &w.vec, nvec))) return rc;
+    if ((rc = dev_alloc(ctx, &w.forced, B * S))) return rc;
+    if ((rc = dev_alloc(ctx, &w.out, B * S))) return rc;
+    if ((rc = dev_alloc(ctx, &w.n_done, B))) return rc;
+    L2B_CUDA(ctx, cudaMemsetAsync(w.counters, 0, B * ctx->heads_loc * sizeof(unsigned int), ctx->stream));
+    void *h = nullptr;
+    L2B_CUDA(ctx, cudaHostAlloc(&h, nvec * sizeof(BatchVec), cudaHostAllocDefault));
+    w.pinned.push_back(h); w.h_vec = static_cast<BatchVec *>(h);
+    L2B_CUDA(ctx, cudaHostAlloc(&h, B * V * sizeof(float), cudaHostAllocDefault));
+    w.pinned.push_back(h); w.h_logits = static_cast<float *>(h);
+    L2B_CUDA(ctx, cudaHostAlloc(&h, (B * S + B) * sizeof(int), cudaHostAllocDefault));
+    w.pinned.push_back(h); w.h_ints = static_cast<int *>(h);
+    L2B_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return L2B_OK;
+}
+
+// can this context run PF_MAXB vectors per weight pass?  Single GPU, flash attention, and all four
+// per-layer GEMVs bandwidth-bound shapes of the TMA-ring kernel; otherwise l2b_prefill runs the
+// positions one by one on the device and the batch calls run each stream's own step in turn (same
+// results, weights streamed once per token).
 static int pf_prepare(l2b_ctx *ctx) {
     if (ctx->pf_ready) return L2B_OK;
     ctx->pf_ready = true;
     const char *env = getenv("L2B_PREFILL_BATCH");
     if (env && env[0] == '0') return L2B_OK;
-    const uint64_t dim = ctx->dim, hid = ctx->hid_loc, q = ctx->q_loc;
+    const uint64_t dim = ctx->dim, hid = ctx->hid_loc;
     size_t smem = 0;
     const bool shapes_ok = ctx->world == 1 && !ctx->leader && dim >= (uint64_t)ctx->big_min_n && hid >= (uint64_t)ctx->big_min_n &&
                            dim <= 5 * (TMA_THREADS - 32) * 4 && ctx->gemv8_min_bytes >= 0 &&
@@ -1610,17 +1693,16 @@ static int pf_prepare(l2b_ctx *ctx) {
                            (kPfSmemBudget - 2 * hid * 4) / ((size_t)TMA_STAGE_FLOATS * 4) >= 2;
     if (!shapes_ok) return L2B_OK;
     L2B_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_x, PF_MAXB * dim))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_q, PF_MAXB * q))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_xb, PF_MAXB * q))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_hb, PF_MAXB * hid))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_part_o, (size_t)PF_MAXB * ctx->heads_loc * ctx->nsplit * ctx->head_size))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_part_ml, (size_t)PF_MAXB * ctx->heads_loc * ctx->nsplit * 2))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_counters, (size_t)PF_MAXB * ctx->heads_loc))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->pf_tokens, (size_t)ctx->cfg.seq_len))) return rc;
-    L2B_CUDA(ctx, cudaMemsetAsync(ctx->pf_counters, 0, (size_t)PF_MAXB * ctx->heads_loc * sizeof(unsigned int), ctx->stream));
-    for (int epi : {(int)EPI_QKV, (int)EPI_SILU, (int)EPI_RESID}) {
+    WeightStore &w = *ctx->weights;
+    if (!w.batch_ready) {
+        const size_t mark = ctx->owned.size();
+        const int rc = alloc_batch_scratch(ctx, w);
+        w.owned.insert(w.owned.end(), ctx->owned.begin() + mark, ctx->owned.end());   // the store frees them
+        ctx->owned.resize(mark);
+        if (rc) return rc;
+        w.batch_ready = true;
+    }
+    for (int epi : {(int)EPI_QKV, (int)EPI_SILU, (int)EPI_RESID, (int)EPI_STORE, (int)EPI_ARGMAX}) {
         L2B_CUDA(ctx, cudaFuncSetAttribute(pf_pick<PF_MAXB>(epi), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPfSmemBudget));
         L2B_CUDA(ctx, cudaFuncSetAttribute(pf_pick<2>(epi), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPfSmemBudget));
     }
@@ -1650,92 +1732,125 @@ static int pf_launch(l2b_ctx *ctx, int epi, PrefillParams p, cudaStream_t st) {
     return L2B_OK;
 }
 
+// Layer l (src/main.zig:305-422) for the n <= L2B_MAX_BATCH vectors vec[0..n) whose residual streams are
+// weights->x[0..n): PF_MAXB vectors per pass over the dim-wide weights, two per pass over w2 (its
+// hidden-wide inputs fill shared memory), one attention launch for all n.  Prompt prefill and batched
+// decode both run their layers through here.
+static int enqueue_batch_layer(l2b_ctx *ctx, cudaStream_t st, int l, const BatchVec *vec, int n) {
+    const l2b_config &c = ctx->cfg;
+    const WeightStore &w = *ctx->weights;
+    const int dim = ctx->dim;
+    const size_t loff = (size_t)l * c.seq_len * ctx->kv_loc;
+    int rc;
+    // ---- rmsnorm + q,k,v + RoPE + KV append (:305-358)
+    for (int g = 0; g < n; g += PF_MAXB) {
+        PrefillParams p{};
+        p.n = dim; p.nb = n - g < PF_MAXB ? n - g : PF_MAXB; p.vec = vec + g;
+        p.x_in = w.x + (size_t)g * dim;
+        if (l == 0) { p.emb = ctx->emb; p.x_out = w.x + (size_t)g * dim; }   // :295-296
+        p.gamma = ctx->rms_att + (size_t)l * dim;
+        p.w0 = ctx->wq + (size_t)l * ctx->q_loc * dim;
+        p.w1 = ctx->wk + (size_t)l * ctx->kv_loc * dim;
+        p.w2 = ctx->wv + (size_t)l * ctx->kv_loc * dim;
+        p.rows0 = ctx->q_loc; p.rows1 = ctx->kv_loc; p.rows2 = ctx->kv_loc;
+        p.total_rows = ctx->q_loc + 2 * ctx->kv_loc;
+        p.out0 = w.q + (size_t)g * ctx->q_loc;
+        p.kv_off = loff;
+        p.rope_cos = ctx->rope_cos; p.rope_sin = ctx->rope_sin;
+        p.head_size = ctx->head_size; p.kv_dim = ctx->kv_loc;
+        if ((rc = pf_launch<PF_MAXB>(ctx, EPI_QKV, p, st))) return rc;
+    }
+    // ---- attention of the n queries (:361-389); query z sees positions 0 .. vec[z].pos of its own cache
+    {
+        size_t attn_smem = 0;
+        attn_fn afn = pick_attention(ctx->head_size, true, &attn_smem);
+        AttnParams a{};
+        a.ctl = ctx->ctl; a.q = w.q; a.vec = vec; a.kv_off = loff;
+        a.xb = w.xb; a.part_o = w.part_o; a.part_ml = w.part_ml; a.counters = w.counters;
+        a.head_size = ctx->head_size; a.kv_dim = ctx->kv_loc; a.kv_mul = ctx->kv_mul;
+        a.nsplit = ctx->nsplit; a.min_chunk = ctx->min_chunk;
+        a.q_stride = ctx->q_loc; a.seq_len = c.seq_len;
+        cudaLaunchConfig_t lc{};
+        lc.gridDim = dim3(ctx->heads_loc, ctx->nsplit, n);
+        lc.blockDim = dim3(NT);
+        lc.dynamicSmemBytes = attn_smem;
+        lc.stream = st;
+        cudaLaunchAttribute at[1] = {pdl_attr()};
+        lc.attrs = at;
+        lc.numAttrs = ctx->use_pdl ? 1 : 0;
+        L2B_CUDA(ctx, cudaLaunchKernelEx(&lc, afn, a));
+        ++ctx->last_launches;
+    }
+    // ---- wo + residual (:392-395)
+    for (int g = 0; g < n; g += PF_MAXB) {
+        PrefillParams o{};
+        o.n = ctx->q_loc; o.nb = n - g < PF_MAXB ? n - g : PF_MAXB; o.vec = vec + g;
+        o.x_in = w.xb + (size_t)g * ctx->q_loc;
+        o.w0 = ctx->wo + (size_t)l * dim * ctx->q_loc;
+        o.total_rows = dim; o.rows0 = dim;
+        o.out0 = w.x + (size_t)g * dim;
+        if ((rc = pf_launch<PF_MAXB>(ctx, EPI_RESID, o, st))) return rc;
+    }
+    // ---- rmsnorm + w1,w3 + SiLU*mul (:398-416)
+    for (int g = 0; g < n; g += PF_MAXB) {
+        PrefillParams f{};
+        f.n = dim; f.nb = n - g < PF_MAXB ? n - g : PF_MAXB; f.vec = vec + g;
+        f.x_in = w.x + (size_t)g * dim;
+        f.gamma = ctx->rms_ffn + (size_t)l * dim;
+        f.w0 = ctx->w1 + (size_t)l * ctx->hid_loc * dim;
+        f.w1 = ctx->w3 + (size_t)l * ctx->hid_loc * dim;
+        f.rows0 = ctx->hid_loc;
+        f.total_rows = 2 * ctx->hid_loc;
+        f.out0 = w.hb + (size_t)g * ctx->hid_loc;
+        if ((rc = pf_launch<PF_MAXB>(ctx, EPI_SILU, f, st))) return rc;
+    }
+    // ---- w2 + residual (:419-422); hidden-sized inputs: two vectors per pass (shared memory)
+    for (int b = 0; b < n; b += 2) {
+        PrefillParams d{};
+        d.n = ctx->hid_loc; d.nb = n - b < 2 ? n - b : 2; d.vec = vec + b;
+        d.x_in = w.hb + (size_t)b * ctx->hid_loc;
+        d.w0 = ctx->w2 + (size_t)l * dim * ctx->hid_loc;
+        d.total_rows = dim; d.rows0 = dim;
+        d.out0 = w.x + (size_t)b * dim;
+        if ((rc = pf_launch<2>(ctx, EPI_RESID, d, st))) return rc;
+    }
+    return L2B_OK;
+}
+
+// final rmsnorm + classifier (:426-429) of the n vectors: logits rows weights->logits[0..n), and with
+// argmax the packed first-maximum key of vector b at weights->amax[b]
+static int enqueue_batch_classifier(l2b_ctx *ctx, cudaStream_t st, const BatchVec *vec, int n, bool argmax) {
+    const WeightStore &w = *ctx->weights;
+    for (int g = 0; g < n; g += PF_MAXB) {
+        PrefillParams k{};
+        k.n = ctx->dim; k.nb = n - g < PF_MAXB ? n - g : PF_MAXB; k.vec = vec + g;
+        k.x_in = w.x + (size_t)g * ctx->dim;
+        k.gamma = ctx->rms_final;
+        k.w0 = ctx->wcls;
+        k.total_rows = ctx->vocab_loc; k.rows0 = ctx->vocab_loc;
+        k.out0 = w.logits + (size_t)g * ctx->vocab_loc;
+        k.amax = w.amax + g;
+        const int rc = pf_launch<PF_MAXB>(ctx, argmax ? EPI_ARGMAX : EPI_STORE, k, st);
+        if (rc) return rc;
+    }
+    return L2B_OK;
+}
+
 // n_tokens positions starting at pos0, PF_MAXB per pass over the weights; KV cache filled, no logits
 static int prefill_batched(l2b_ctx *ctx, const int32_t *tokens, int n_tokens, int pos0) {
     const l2b_config &c = ctx->cfg;
-    const int dim = ctx->dim;
+    WeightStore &w = *ctx->weights;
     cudaStream_t st = ctx->stream;
     L2B_CUDA(ctx, cudaSetDevice(ctx->device));
-    for (int i = 0; i < n_tokens; ++i) ctx->h_gen[i] = tokens[i];
-    L2B_CUDA(ctx, cudaMemcpyAsync(ctx->pf_tokens, ctx->h_gen, (size_t)n_tokens * sizeof(int), cudaMemcpyHostToDevice, st));
-    fill_ctl(ctx, tokens[0], pos0, 0, 1.0f, -1.0f);          // DONE = 0 for the attention kernel
-    L2B_CUDA(ctx, cudaMemcpyAsync(ctx->ctl, ctx->h_ctl, CTL_HOST_WORDS * sizeof(int), cudaMemcpyHostToDevice, st));
+    for (int i = 0; i < n_tokens; ++i) w.h_vec[i] = BatchVec{tokens[i], pos0 + i, 0, 0, 1, 0, ctx->kcache, ctx->vcache};
+    L2B_CUDA(ctx, cudaMemcpyAsync(w.vec, w.h_vec, (size_t)n_tokens * sizeof(BatchVec), cudaMemcpyHostToDevice, st));
     L2B_CUDA(ctx, cudaEventRecord(ctx->ev0, st));
     ctx->last_launches = 0;
-    size_t attn_smem = 0;
-    attn_fn afn = pick_attention(ctx->head_size, true, &attn_smem);
     for (int done = 0; done < n_tokens; done += PF_MAXB) {
         const int nb = n_tokens - done < PF_MAXB ? n_tokens - done : PF_MAXB;
-        const int pos = pos0 + done;
         for (int l = 0; l < c.n_layers; ++l) {
-            // ---- rmsnorm + q,k,v + RoPE + KV append for nb positions (:305-358)
-            PrefillParams p{};
-            p.n = dim; p.nb = nb; p.pos0 = pos;
-            p.x_in = ctx->pf_x;
-            if (l == 0) { p.emb = ctx->emb; p.tokens = ctx->pf_tokens + done; p.x_out = ctx->pf_x; }
-            p.gamma = ctx->rms_att + (size_t)l * dim;
-            p.w0 = ctx->wq + (size_t)l * ctx->q_loc * dim;
-            p.w1 = ctx->wk + (size_t)l * ctx->kv_loc * dim;
-            p.w2 = ctx->wv + (size_t)l * ctx->kv_loc * dim;
-            p.rows0 = ctx->q_loc; p.rows1 = ctx->kv_loc; p.rows2 = ctx->kv_loc;
-            p.total_rows = ctx->q_loc + 2 * ctx->kv_loc;
-            p.out0 = ctx->pf_q;
-            const size_t loff = (size_t)l * c.seq_len * ctx->kv_loc;
-            p.kcache = ctx->kcache + loff;
-            p.vcache = ctx->vcache + loff;
-            p.rope_cos = ctx->rope_cos; p.rope_sin = ctx->rope_sin;
-            p.head_size = ctx->head_size; p.kv_dim = ctx->kv_loc;
-            int rc = pf_launch<PF_MAXB>(ctx, EPI_QKV, p, st);
+            const int rc = enqueue_batch_layer(ctx, st, l, w.vec + done, nb);
             if (rc) return rc;
-            // ---- attention of the nb queries (:361-389); query z sees positions 0 .. pos+z
-            AttnParams a{};
-            a.ctl = ctx->ctl; a.q = ctx->pf_q; a.kcache = ctx->kcache + loff; a.vcache = ctx->vcache + loff;
-            a.xb = ctx->pf_xb; a.part_o = ctx->pf_part_o; a.part_ml = ctx->pf_part_ml; a.counters = ctx->pf_counters;
-            a.head_size = ctx->head_size; a.kv_dim = ctx->kv_loc; a.kv_mul = ctx->kv_mul;
-            a.nsplit = ctx->nsplit; a.min_chunk = ctx->min_chunk;
-            a.pos_base = pos; a.q_stride = ctx->q_loc; a.seq_len = c.seq_len;
-            cudaLaunchConfig_t lc{};
-            lc.gridDim = dim3(ctx->heads_loc, ctx->nsplit, nb);
-            lc.blockDim = dim3(NT);
-            lc.dynamicSmemBytes = attn_smem;
-            lc.stream = st;
-            cudaLaunchAttribute at[1] = {pdl_attr()};
-            lc.attrs = at;
-            lc.numAttrs = ctx->use_pdl ? 1 : 0;
-            L2B_CUDA(ctx, cudaLaunchKernelEx(&lc, afn, a));
-            ++ctx->last_launches;
-            // ---- wo + residual (:392-395)
-            PrefillParams o{};
-            o.n = ctx->q_loc; o.nb = nb; o.pos0 = pos;
-            o.x_in = ctx->pf_xb;
-            o.w0 = ctx->wo + (size_t)l * dim * ctx->q_loc;
-            o.total_rows = dim; o.rows0 = dim;
-            o.out0 = ctx->pf_x;
-            rc = pf_launch<PF_MAXB>(ctx, EPI_RESID, o, st);
-            if (rc) return rc;
-            // ---- rmsnorm + w1,w3 + SiLU*mul (:398-416)
-            PrefillParams f{};
-            f.n = dim; f.nb = nb; f.pos0 = pos;
-            f.x_in = ctx->pf_x;
-            f.gamma = ctx->rms_ffn + (size_t)l * dim;
-            f.w0 = ctx->w1 + (size_t)l * ctx->hid_loc * dim;
-            f.w1 = ctx->w3 + (size_t)l * ctx->hid_loc * dim;
-            f.rows0 = ctx->hid_loc;
-            f.total_rows = 2 * ctx->hid_loc;
-            f.out0 = ctx->pf_hb;
-            rc = pf_launch<PF_MAXB>(ctx, EPI_SILU, f, st);
-            if (rc) return rc;
-            // ---- w2 + residual (:419-422); hidden-sized inputs: two positions per pass (shared memory)
-            for (int b = 0; b < nb; b += 2) {
-                PrefillParams d{};
-                d.n = ctx->hid_loc; d.nb = nb - b < 2 ? nb - b : 2; d.pos0 = pos + b;
-                d.x_in = ctx->pf_hb + (size_t)b * ctx->hid_loc;
-                d.w0 = ctx->w2 + (size_t)l * dim * ctx->hid_loc;
-                d.total_rows = dim; d.rows0 = dim;
-                d.out0 = ctx->pf_x + (size_t)b * dim;
-                rc = pf_launch<2>(ctx, EPI_RESID, d, st);
-                if (rc) return rc;
-            }
         }
     }
     L2B_CUDA(ctx, cudaEventRecord(ctx->ev1, st));
@@ -1743,6 +1858,99 @@ static int prefill_batched(l2b_ctx *ctx, const int32_t *tokens, int n_tokens, in
     L2B_CUDA(ctx, cudaGetLastError());
     L2B_CUDA(ctx, cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
     if (pos0 + n_tokens > ctx->n_appended) ctx->n_appended = pos0 + n_tokens;
+    return L2B_OK;
+}
+
+// Decode steps of n streams over one set of weights, every pass over the weights shared by up to
+// PF_MAXB of them, on streams[0]'s CUDA stream.  host_logits != nullptr: one step, logits [n][vocab]
+// returned.  Otherwise the temperature-0 loop of l2b_generate_argmax for every stream at once: stream k
+// takes min(n_steps, seq_len - pos[k]) steps, its tokens chosen by advance_batch_kernel on the device.
+static int run_batch(l2b_ctx *const *streams, int n, const int32_t *tokens, const int32_t *pos, int n_steps,
+                     const int32_t *forced, int stop_on_bos, float *host_logits, int32_t *out_next, int32_t *n_done) {
+    l2b_ctx *lead = streams[0];
+    WeightStore &w = *lead->weights;
+    cudaStream_t st = lead->stream;
+    const size_t S = lead->cfg.seq_len, V = lead->cfg.vocab_size, B = L2B_MAX_BATCH;
+    const bool gen = host_logits == nullptr;
+    int max_steps = 0;
+    for (int k = 0; k < n; ++k) {
+        const int room = (int)S - pos[k];
+        const int lim = gen ? (n_steps < room ? n_steps : room) : 1;
+        w.h_vec[k] = BatchVec{tokens[k], pos[k], lim > 0 ? 0 : 1, 0, lim, 0, streams[k]->kcache, streams[k]->vcache};
+        if (lim > max_steps) max_steps = lim;
+        for (int i = 0; gen && i < lim; ++i) w.h_ints[k * S + i] = forced ? forced[(size_t)k * n_steps + i] : -1;
+    }
+    if (max_steps == 0) {
+        for (int k = 0; k < n; ++k) n_done[k] = 0;
+        return L2B_OK;
+    }
+    L2B_CUDA(lead, cudaSetDevice(lead->device));
+    L2B_CUDA(lead, cudaMemcpyAsync(w.vec, w.h_vec, (size_t)n * sizeof(BatchVec), cudaMemcpyHostToDevice, st));
+    if (gen) {
+        L2B_CUDA(lead, cudaMemcpyAsync(w.forced, w.h_ints, (size_t)n * S * sizeof(int), cudaMemcpyHostToDevice, st));
+        L2B_CUDA(lead, cudaMemsetAsync(w.n_done, 0, (size_t)n * sizeof(int), st));
+        L2B_CUDA(lead, cudaMemsetAsync(w.amax, 0, (size_t)n * sizeof(unsigned long long), st));
+    }
+    L2B_CUDA(lead, cudaEventRecord(lead->ev0, st));
+    lead->last_launches = 0;
+    int rc;
+    for (int i = 0; i < max_steps; ++i) {
+        for (int l = 0; l < lead->cfg.n_layers; ++l)
+            if ((rc = enqueue_batch_layer(lead, st, l, w.vec, n))) return rc;
+        if ((rc = enqueue_batch_classifier(lead, st, w.vec, n, gen))) return rc;
+        if (gen) {
+            BatchVec *vec = w.vec;
+            unsigned long long *amax = w.amax;
+            const int *fp = w.forced;
+            int *op = w.out, *dp = w.n_done, stride = (int)S, sob = stop_on_bos ? 1 : 0;
+            void *args[] = {&vec, &n, &amax, &fp, &op, &dp, &stride, &sob};
+            if ((rc = launch_small(lead, (const void *)advance_batch_kernel, dim3(1), dim3(32), args, st, true))) return rc;
+        }
+    }
+    if (gen) {
+        L2B_CUDA(lead, cudaMemcpyAsync(w.h_ints, w.out, (size_t)n * S * sizeof(int), cudaMemcpyDeviceToHost, st));
+        L2B_CUDA(lead, cudaMemcpyAsync(w.h_ints + B * S, w.n_done, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st));
+    } else {
+        L2B_CUDA(lead, cudaMemcpyAsync(w.h_logits, w.logits, (size_t)n * V * sizeof(float), cudaMemcpyDeviceToHost, st));
+    }
+    L2B_CUDA(lead, cudaEventRecord(lead->ev1, st));
+    L2B_CUDA(lead, cudaStreamSynchronize(st));
+    L2B_CUDA(lead, cudaGetLastError());
+    L2B_CUDA(lead, cudaEventElapsedTime(&lead->last_ms, lead->ev0, lead->ev1));
+    for (int k = 0; k < n; ++k) {
+        const int steps = gen ? w.h_ints[B * S + k] : 1;
+        if (gen) {
+            n_done[k] = steps;
+            for (int i = 0; i < steps; ++i) out_next[(size_t)k * n_steps + i] = w.h_ints[k * S + i];
+        }
+        if (pos[k] + steps > streams[k]->n_appended) streams[k]->n_appended = pos[k] + steps;
+    }
+    if (!gen) memcpy(host_logits, w.h_logits, (size_t)n * V * sizeof(float));
+    return L2B_OK;
+}
+
+// argument checks of the batch calls (before any CUDA call); errors land on streams[0] when there is one
+static int check_batch_args(l2b_ctx *const *streams, int n, const int32_t *tokens, const int32_t *pos) {
+    if (!streams || !tokens || !pos) { g_create_error = "NULL argument"; return L2B_ERR_INVALID_ARG; }
+    if (n < 1 || n > L2B_MAX_BATCH) {
+        g_create_error = "n must be 1 .. L2B_MAX_BATCH";
+        return fail(n > 0 ? streams[0] : nullptr, L2B_ERR_INVALID_ARG, "n must be 1 .. L2B_MAX_BATCH");
+    }
+    for (int k = 0; k < n; ++k)
+        if (!streams[k]) { g_create_error = "NULL stream"; return fail(streams[0], L2B_ERR_INVALID_ARG, "NULL stream"); }
+    for (int k = 0; k < n; ++k) {
+        for (int j = 0; j < k; ++j)
+            if (streams[j] == streams[k]) return fail(streams[0], L2B_ERR_INVALID_ARG, "the same stream is listed twice");
+        if (!streams[k]->weights || streams[k]->weights != streams[0]->weights)
+            return fail(streams[0], L2B_ERR_INVALID_ARG, "streams over different weights");
+    }
+    for (int k = 0; k < n; ++k) {
+        const int rc = check_step_args(streams[k], tokens[k], pos[k]);
+        if (rc) {
+            if (k) streams[0]->err = "stream " + std::to_string(k) + ": " + streams[k]->err;
+            return rc;
+        }
+    }
     return L2B_OK;
 }
 
@@ -1848,6 +2056,74 @@ int32_t l2b_prefill(l2b_ctx *ctx, const int32_t *tokens, int32_t n_tokens, int32
         if (done != n_silent) return fail(ctx, L2B_ERR_STATE, "prefill stopped early");
     }
     if (host_logits) return l2b_forward(ctx, tokens[n_tokens - 1], pos0 + n_tokens - 1, host_logits);
+    return L2B_OK;
+}
+
+// ---- decode streams over one copy of the weights --------------------------------------------------
+int32_t l2b_create_stream(l2b_ctx **out, l2b_ctx *base) {
+    if (!out || !base) { g_create_error = "NULL argument"; return L2B_ERR_INVALID_ARG; }
+    *out = nullptr;
+    if (base->world > 1 || base->leader || !base->members.empty() || !base->weights) {
+        g_create_error = "decode streams share the weights of a single-GPU context only";
+        return fail(base, L2B_ERR_UNSUPPORTED, "decode streams share the weights of a single-GPU context only");
+    }
+    l2b_ctx *ctx = new l2b_ctx();
+    int rc = open_rank(ctx, &base->cfg, 0, 1, base->device, base->num_sms);
+    if (rc == L2B_OK) {
+        ctx->weights = base->weights;       // no upload: load_bytes stays 0
+        ctx->emb = base->emb; ctx->rms_att = base->rms_att; ctx->rms_ffn = base->rms_ffn; ctx->rms_final = base->rms_final;
+        ctx->wq = base->wq; ctx->wk = base->wk; ctx->wv = base->wv; ctx->wo = base->wo;
+        ctx->w1 = base->w1; ctx->w2 = base->w2; ctx->w3 = base->w3; ctx->wcls = base->wcls;
+        rc = init_run_state(ctx, nullptr, nullptr, base);
+    }
+    if (rc == L2B_OK) rc = warm_up(std::vector<l2b_ctx *>{ctx});
+    if (rc) {
+        destroy_rank(ctx);
+        return rc;
+    }
+    *out = ctx;
+    return L2B_OK;
+}
+
+int32_t l2b_forward_batch(l2b_ctx *const *streams, int32_t n, const int32_t *tokens, const int32_t *pos,
+                          float *host_logits) {
+    int rc = check_batch_args(streams, n, tokens, pos);
+    if (rc) return rc;
+    l2b_ctx *lead = streams[0];
+    if (!host_logits) return fail(lead, L2B_ERR_INVALID_ARG, "host_logits is NULL");
+    if ((rc = pf_prepare(lead))) return rc;
+    if (lead->pf_ok) return run_batch(streams, n, tokens, pos, 1, nullptr, 0, host_logits, nullptr, nullptr);
+    // latency-bound shapes: each stream's own step in turn
+    const size_t V = lead->cfg.vocab_size;
+    float ms = 0.0f;
+    int launches = 0;
+    for (int k = 0; k < n; ++k) {
+        rc = l2b_forward(streams[k], tokens[k], pos[k], host_logits + (size_t)k * V);
+        if (rc) { if (k) lead->err = streams[k]->err; return rc; }
+        ms += streams[k]->last_ms; launches += streams[k]->last_launches;
+    }
+    lead->last_ms = ms; lead->last_launches = launches;
+    return L2B_OK;
+}
+
+int32_t l2b_generate_argmax_batch(l2b_ctx *const *streams, int32_t n, const int32_t *tokens, const int32_t *pos,
+                                  int32_t n_steps, const int32_t *forced, int32_t stop_on_bos, int32_t *out_next,
+                                  int32_t *n_done) {
+    int rc = check_batch_args(streams, n, tokens, pos);
+    if (rc) return rc;
+    l2b_ctx *lead = streams[0];
+    if (!out_next || !n_done || n_steps < 0) return fail(lead, L2B_ERR_INVALID_ARG, "bad generate arguments");
+    if ((rc = pf_prepare(lead))) return rc;
+    if (lead->pf_ok) return run_batch(streams, n, tokens, pos, n_steps, forced, stop_on_bos, nullptr, out_next, n_done);
+    float ms = 0.0f;
+    int launches = 0;
+    for (int k = 0; k < n; ++k) {
+        rc = l2b_generate_argmax(streams[k], tokens[k], pos[k], n_steps, forced ? forced + (size_t)k * n_steps : nullptr,
+                                 stop_on_bos, out_next + (size_t)k * n_steps, &n_done[k]);
+        if (rc) { if (k) lead->err = streams[k]->err; return rc; }
+        if (n_done[k] > 0) { ms += streams[k]->last_ms; launches += streams[k]->last_launches; }
+    }
+    lead->last_ms = ms; lead->last_launches = launches;
     return L2B_OK;
 }
 
@@ -2132,7 +2408,7 @@ int32_t l2b_op_attention_head(int32_t device, float *out, const float *q, const 
     a.ctl = ctl; a.q = dq; a.kcache = dk; a.vcache = dv; a.xb = dout; a.part_o = po; a.part_ml = pml;
     a.counters = cnt; a.head_size = head_size; a.kv_dim = kv_stride; a.kv_mul = 1; a.nsplit = nsplit;
     a.min_chunk = 64;
-    a.pos_base = -1;
+    a.vec = nullptr;                 // single position from the control block
     a.seq_len = n_pos;
     int cap = (n_pos + nsplit - 1) / nsplit;
     if (cap < 64) cap = 64;
